@@ -7,7 +7,7 @@ sweep (115 200 rays) = 1 497 600 traced rays, reference default grids / MLPs (ra
 Metric as the reference defines it: rays / time between device synchronisations (nerfstudio/pipelines/ad_pipeline.py:
 198-208, 296-304); only TRACED rays are counted (the reference counts the 9x larger full-resolution pixel grid).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Two timed arms per run:
   value  device-resident inputs: ray generation + ONE `get_nff_outputs` launch pair over the whole time step.
@@ -78,6 +78,16 @@ ALGO_BYTES_PER_RAY = 69_900  # SURVEY.md section 8(d) / BASELINE.md section 2: f
 CAM_RAYS = 640 * 360
 WORKLOAD = "neurad-default config2: 6x1920x1080 pinhole @stride3 (6x230400 rays) + 64x1800 lidar (115200 rays), 0 actors"
 STRONG_RAYS = 8_388_608  # BASELINE configs[4]
+DUMP_ROWS = 131_072  # --dump-outputs keeps at most this many rows of an output (48-wide features: 25 MB)
+
+
+def sample_rows(t: torch.Tensor):
+    """`t` as [rows, channels] float32 numpy; above DUMP_ROWS rows, a fixed seeded sample of them (in order)."""
+    t = t.reshape(-1, t.shape[-1])
+    if t.shape[0] > DUMP_ROWS:
+        keep = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+        t = t[keep.to(t.device)]
+    return t.float().cpu().numpy()
 
 
 def measured_peaks():
@@ -420,7 +430,15 @@ def main():
     ap.add_argument("--gather", default="p2p", choices=["p2p", "nccl"],
                     help="N>1: p2p = render epilogue stores rows into every peer's buffer over NVLink (default); "
                          "nccl = all_gather_into_tensor after the render")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned to DIR/<name>.npy (float32): render_* the "
+                         "device-resident arm's outputs, camera_* / lidar_* the API arm's host buffers (a fixed sample of "
+                         f"{DUMP_ROWS} rows where an output has more); rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -525,6 +543,9 @@ def main():
         sampler.start()
     step.launches = 0
     ms = timed(lambda: step.run_device(True), args.steps)
+    dump = {}
+    if args.dump_outputs and rank == 0:
+        dump = {f"render_{k}": sample_rows(v) for k, v in dict({k: b[rank] for k, b in step.gather.items()}, **step.local).items()}
     launches = step.launches // args.steps
     kern_ms = sorted(a.elapsed_time(b) for a, b in step.kernel_events)
     kern_ms = sum(kern_ms) / len(kern_ms)
@@ -536,6 +557,9 @@ def main():
     if dec_stream:
         model.set_decoder_stream(torch.cuda.Stream(device=dev))
     ms_e2e = timed(step.run_e2e, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump.update({f"camera_{k}": sample_rows(torch.stack([h[k] for h in step.host_cam])) for k in step.host_cam[0]})
+        dump.update({f"lidar_{k}": sample_rows(v) for k, v in step.host_lidar.items()})
     e2e_launches = step.e2e_launches // args.steps
     # the host buffers the e2e arm filled must hold what the API returns on the device (last image + the sweep re-rendered)
     if step.p2p:
@@ -591,9 +615,8 @@ def main():
 
         for _ in range(2):
             run_strong()
-        k_strong = max(2, args.steps // 3)
-        ms_s = timed(run_strong, k_strong)
-        strong = {"rays_total": per * world, "rays_per_gpu": per, "ms_per_batch": ms_s / k_strong, "value": per * world / (ms_s / k_strong * 1e-3),
+        ms_s = timed(run_strong, args.steps)
+        strong = {"rays_total": per * world, "rays_per_gpu": per, "ms_per_batch": ms_s / args.steps, "value": per * world / (ms_s / args.steps * 1e-3),
                   "unit": "rays/s", "scaling": "strong", "what": "BASELINE configs[4]: one 8 388 608-ray batch (config-2 rays repeated), contiguous 1/N shards, fused peer-store gather"}
         be.set_peer_outputs(None)
         del big, sout
@@ -683,6 +706,12 @@ def main():
         v, n, dt = oracle_rays_per_sec(cfg, args.cpu_sample)
         line["cpu_baseline"] = {"value": v, "unit": "rays/s", "cores": torch.get_num_threads(), "kind": "port",
                                 "sample": f"{n} rays (12:1 camera:lidar; render + lidar head + rgb decoder) of the same workload in {dt:.1f} s, oracle port of the reference torch path, best of thread counts probed, host has {os.cpu_count()} cpus"}
+    if args.dump_outputs:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     _emit(line)
     if world > 1:
         import torch.distributed as dist
@@ -762,11 +791,10 @@ def secondary_legs(be, cfg, dev, steps, timed) -> dict:
         for _ in range(3):
             run4()
         ev.clear()
-        k_steps = steps * 4
-        ms4 = timed(run4, k_steps)
+        ms4 = timed(run4, steps)
         be.check_status()
         k4 = sum(a.elapsed_time(b) for a, b in ev) / len(ev)
-        out["config4_lidar_grid"] = {"value": n4 * k_steps / (ms4 * 1e-3), "unit": "rays/s", "ms_per_sweep": ms4 / k_steps, "rays_per_sweep": n4,
+        out["config4_lidar_grid"] = {"value": n4 * steps / (ms4 * 1e-3), "unit": "rays/s", "ms_per_sweep": ms4 / steps, "rays_per_sweep": n4,
                                      "roofline": roofline_block(n4, k4, "nff_sample_lane_kernel + nff_shade_lane_kernel + lidar_decode_kernel, 262 144 rays"),
                                      "what": "BASELINE configs[3] (SURVEY 8d reading): 128-beam x 2048-azimuth sweep, per-ray time offset over the 0.1 s revolution, origin + velocity * dt, rendered through the volumetric path + lidar head"}
         del rays, res

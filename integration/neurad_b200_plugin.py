@@ -14,8 +14,9 @@ loop (`neurad.py:650-659`), and in eval mode the rgb / lidar decoders run on the
 the reference's own `nn.Parameter`s in the `implementation="torch"` layout (bound zero-copy by pointer), so checkpoints,
 optimizers and `state_dict()` are untouched.  Training (grad mode) falls through to the reference's own module walk.
 
-Nothing in `neurad-studio_b200/` imports this file; `tests/test_reference_plugin.py` drives it against the real reference
-in the build container (model built by the reference's own config system, dispatch through `discover_methods()`).
+Nothing in `neurad-studio_b200/` imports this file; `oracle/make_golden_reference_recipe.py` builds its model through the
+reference's own config system and `discover_methods()` and checks it against the reference's torch path before writing
+the golden data of `tests/test_reference_recipe.py`.
 """
 from __future__ import annotations
 

@@ -30,7 +30,7 @@ _STUBS = [
 
 
 # further absent third-party packages that only the FULL method registry (nerfstudio.configs.method_configs: every
-# dataparser and model of the reference) pulls in; needed by tests/test_reference_plugin.py, not by the golden generators
+# dataparser and model of the reference) pulls in; needed by oracle/make_golden_reference_recipe.py
 _STUBS_FULL = [
     "av2", "av2.utils", "av2.utils.io", "av2.datasets", "av2.datasets.sensor", "av2.datasets.sensor.av2_sensor_dataloader",
     "av2.datasets.sensor.constants", "av2.geometry", "av2.geometry.geometry", "av2.structures", "av2.structures.sweep",
